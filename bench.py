@@ -4,6 +4,9 @@
   python bench.py [--gpus N] [--steps K] [--warmup W]        # own arm (CUDA, libowwb200)
   python bench.py --impl reference [...]                    # reference arm (CPU, host cores)
   torchrun --nproc-per-node N ... bench.py --gpus N ...      # one rank per GPU, weak scaling
+  python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs as DIR/*.npy
+
+The library is loaded as __graft_entry__.build() left it; the benchmark compiles and writes nothing in the tree.
 
 Headline workload = configs[2]: 8192 concurrent synthetic 16 kHz streams per GPU, 80 ms frames, all six pre-trained
 wake-word head shapes (alexa, hey_mycroft, hey_jarvis [two networks + verifier gate], hey_rhasspy, weather:
@@ -37,6 +40,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: no __pycache__ next to the sources
 
 FLOPS_PER_WINDOW = 2 * 41955840          # SURVEY.md Appendix B (reference-algorithmic, per 76x32 window)
 EXEC_FLOPS_PER_FRAME = 2 * 5612544       # what the incremental path computes per frame with one MMA term per K step (SURVEY.md F10)
@@ -177,9 +181,9 @@ def _cpu_worker(conn, stream_id, seed, workload):
         # in this image - SURVEY.md F2 - but the arm upgrades itself when the assets exist)
         try:
             import glob
-            for extra in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-                if os.path.isdir(extra) and extra not in sys.path:
-                    sys.path.insert(0, extra)
+            extra = os.path.join(ROOT, "baseline", "_ref")
+            if os.path.isdir(extra) and extra not in sys.path:
+                sys.path.insert(0, extra)
             import openwakeword
             hp = sorted(p for p in glob.glob(os.path.join(where, "*.onnx"))
                         if os.path.basename(p) not in ("melspectrogram.onnx", "embedding_model.onnx", "silero_vad.onnx"))
@@ -374,7 +378,7 @@ def measure(args, wl, rank, world, local, dev, sampler_windows, do_model=True):
     t_a = time.perf_counter()
     e0.record()
     for k in range(K):
-        sh.step(dev_steps[(Wm + k) % POOL], 1)
+        scores = sh.step(dev_steps[(Wm + k) % POOL], 1)
     sh.flush()
     e1.record()
     barrier()
@@ -383,6 +387,11 @@ def measure(args, wl, rank, world, local, dev, sampler_windows, do_model=True):
     stage = eng.ctx.stage_ms()
     eng.ctx.enable_stage_timing(0)
     launches = eng.ctx.launch_count - l0
+    dump = {}                                   # name -> what the caller of a timed path received in its last step
+    if args.dump_outputs and rank == 0:
+        if isinstance(scores, owd.GatheredScores):
+            scores = scores.wait()
+        dump[f"{wl}_step"] = scores.cpu().numpy()
     # ---- timed region 2: end to end through the host-buffer C-ABI call (two tickets in flight) ----
     h_scores = np.empty((B, eng.n_cols), np.float32)
     for k in range(Wm):
@@ -393,16 +402,19 @@ def measure(args, wl, rank, world, local, dev, sampler_windows, do_model=True):
     for k in range(1, K + 1):
         nxt = eng.submit(host_steps[(Wm + k) % POOL], 1) if k < K else None
         eng.collect(ticket, h_scores)
+        gathered = h_scores
         if world > 1:
-            owd.gather_scores(torch.from_numpy(h_scores).to(dev), n_total)
+            gathered = owd.gather_scores(torch.from_numpy(h_scores).to(dev), n_total)
         ticket = nxt
     torch.cuda.synchronize()
     t1 = time.perf_counter()
     sampler_windows.append((t0, t1))
     ms_e2e = 1e3 * (t1 - t0)
+    if args.dump_outputs and rank == 0:
+        dump[f"{wl}_step_host"] = gathered.cpu().numpy() if world > 1 else gathered.copy()
     out = {"B": B, "ms_dev": ms_dev, "ms_e2e": ms_e2e, "cnn_ms": stage["cnn"], "heads_ms": stage["heads"], "mel_ms": stage["mel"],
            "launches": int(launches), "n_cols": eng.n_cols, "heads": len(heads), "G": None, "gather": sh.gather_kind,
-           "h2d": B * CHUNK * 2, "d2h": B * eng.n_cols * 4}
+           "h2d": B * CHUNK * 2, "d2h": B * eng.n_cols * 4, "dump": dump}
     # ---- parity of the configuration that was just timed (rank 0, checker only) ----
     if rank == 0:
         out["parity"] = parity_check(eng, heads, B)
@@ -423,6 +435,8 @@ def measure(args, wl, rank, world, local, dev, sampler_windows, do_model=True):
         sampler_windows.append((t0, t1))
         out["ms_model"] = 1e3 * (t1 - t0)
         out["n_labels"] = len(r)
+        if args.dump_outputs:
+            dump.update({f"{wl}_predict_{label}": v for label, v in r.items()})
         del m
     del sh, eng
     torch.cuda.empty_cache()
@@ -434,7 +448,7 @@ def measure_variant(args, wl, local, dev, split_from, sampler_windows):
     import torch
     from openwakeword_b200.engine import StreamEngine
     B = WORKLOADS[wl]["streams"]
-    K = min(args.steps, 20)
+    K = args.steps
     heads = bench_heads(wl)
     POOL = max(4, int(np.ceil(168e6 / (B * CHUNK * 2))))
     eng = StreamEngine(list(heads.values()), B, embedding="synthetic:0", device_index=local, max_chunks=1, cnn_mode=3, split_from=split_from)
@@ -453,21 +467,22 @@ def measure_variant(args, wl, local, dev, split_from, sampler_windows):
     torch.cuda.synchronize()
     sampler_windows.append((t_a, time.perf_counter()))
     ms = e0.elapsed_time(e1) / K
+    dump = {f"{wl}_split{split_from}_step": out.cpu().numpy()} if args.dump_outputs else {}
     par = parity_check(eng, heads, B)
     del eng
     torch.cuda.empty_cache()
     return {"split_from": split_from, "value": B / (ms * 1e-3), "unit": UNIT, "ms_per_step": ms, "steps": K,
             "parity_max_abs_delta": par["max_abs_delta"], "parity_ok": par["ok"],
             "what": ("conv layers >= %d on fp16 hi/lo split operands" % split_from) if split_from < 20 else
-                    "plain fp16 operands in every conv layer: the whole step in one launch"}
+                    "plain fp16 operands in every conv layer: the whole step in one launch"}, dump
 
 
 def run_own_arm(args):
     import torch
     import torch.distributed as dist
     from openwakeword_b200 import distributed as owd
-    import __graft_entry__ as g
-    g.build()
+    from openwakeword_b200 import _native
+    _native.load_library()                     # as build() left it: a missing library is an error, not a rebuild
     from oracle.probe import parity_label      # labelling only (which oracle the 1e-3 gate was checked against)
 
     rank, world, local = owd.init_process_group("nccl" if int(os.environ.get("WORLD_SIZE", "1")) > 1 else None)
@@ -489,11 +504,17 @@ def run_own_arm(args):
         res[wl] = measure(args, wl, rank, world, local, dev, windows, do_model=(wl == args.workload))
     # other points of the precision / speed curve of cnn_mode 3 (device-resident timing + the same parity gate), 1 GPU only
     variants = []
+    dump = {k: a for wl in order for k, a in res[wl]["dump"].items()}
     if args.variants and world == 1 and args.cnn_mode == 3 and not args.split_from:
         for sf in (15, 20):
-            v = measure_variant(args, args.workload, local, dev, sf, windows)
+            v, d = measure_variant(args, args.workload, local, dev, sf, windows)
             variants.append(v)
+            dump.update(d)
     clocks = sampler.stop(windows) if rank == 0 else None
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(a, np.float32))
 
     keys = ["ms_dev", "ms_e2e", "cnn_ms", "heads_ms", "mel_ms"]
     flat = [res[wl][k] for wl in order for k in keys]
@@ -634,7 +655,12 @@ def main():
     ap.add_argument("--split-from", type=int, default=0,
                     help="first conv layer on fp16 hi/lo split operands (11 = default, scores within ~2e-4 of the fp32 graph; "
                          "20 = plain fp16 everywhere and the whole step as one fused launch, ~9e-4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the scores each timed path returned in its last step as DIR/<name>.npy "
+                         "(float32; inputs are seeded, so runs with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_own_arm(args)

@@ -1,8 +1,8 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference plumbing.
 
-Run in the build container only (needs /root/reference):
-    python tests/golden/make_golden.py
-/root/reference/openwakeword is imported with ``oracle.ref_stub_ort`` standing in
+Needs a checkout of the original openWakeWord project (its ``openwakeword`` package and ``tests/data/*.wav``):
+    python tests/golden/make_golden.py <openWakeWord checkout> [--only-new]
+Its ``openwakeword`` package is imported with ``oracle.ref_stub_ort`` standing in
 for onnxruntime (absent here, SURVEY.md F2), so buffers, windowing, chunk
 accumulation and score post-processing are the reference's own code while the
 three graphs are evaluated by oracle/{mel,embedding,heads}.py on synthetic seeded
@@ -10,6 +10,7 @@ weights (regenerated from the recorded seeds, not stored).  The unseeded
 ``np.random`` state the reference puts in ``feature_buffer`` (SURVEY.md F6) is
 captured and stored as ``feature_init``.
 """
+import argparse
 import os
 import sys
 import tempfile
@@ -42,13 +43,17 @@ def read_wav(path):
 
 
 def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("reference", help="checkout of the original openWakeWord project")
+    ap.add_argument("--only-new", action="store_true", help="keep the committed round-1 fixtures byte-identical")
+    args = ap.parse_args()
     out_dir = os.path.dirname(os.path.abspath(__file__))
     emb = W.synthetic_embedding(EMB_SEED)
     heads = {k: W.synthetic_head(**v) for k, v in HEAD_SPECS.items()}
     heads.update({k: W.synthetic_gated_head(**v) for k, v in GATED_SPECS.items()})
-    only_new = "--only-new" in sys.argv           # keep the committed round-1 fixtures byte-identical
+    only_new = args.only_new
     ref_stub_ort.install(emb, heads)
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, os.path.abspath(args.reference))
     from openwakeword.model import Model            # the reference, unmodified
 
     tmp = tempfile.mkdtemp()
@@ -68,7 +73,7 @@ def main():
             m.class_mapping["timer_v0.1"] = dict(TIMER_MAP)
         return m, m.preprocessor.feature_buffer.astype(np.float32).copy()
 
-    wavs = {n: read_wav(f"/root/reference/tests/data/{n}.wav")
+    wavs = {n: read_wav(os.path.join(args.reference, "tests", "data", n + ".wav"))
             for n in ("alexa_test", "hey_mycroft_test", "hey_jane")}
     cases = {}
 

@@ -1,6 +1,6 @@
 """Generate tests/golden/metrics.npz from the UNMODIFIED reference functions
-(/root/reference/openwakeword/metrics.py).  Run in the build container only:
-    python tests/golden/make_metrics_golden.py
+(openwakeword/metrics.py of the original openWakeWord project):
+    python tests/golden/make_metrics_golden.py <openWakeWord checkout>
 Series are built so that the reference does not raise (its grouping loop indexes one past a transition's 1, so a
 series whose final element is a fresh 0->1 rise makes it throw IndexError)."""
 import importlib.util
@@ -9,9 +9,12 @@ import sys
 
 import numpy as np
 
-spec = importlib.util.spec_from_file_location("ref_metrics", "/root/reference/openwakeword/metrics.py")
-ref = importlib.util.module_from_spec(spec)
-spec.loader.exec_module(ref)
+
+def load_reference_metrics(checkout):
+    spec = importlib.util.spec_from_file_location("ref_metrics", os.path.join(checkout, "openwakeword", "metrics.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
 
 
 def series(rng, kind, T):
@@ -32,6 +35,9 @@ def series(rng, kind, T):
 
 
 def main():
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    ref = load_reference_metrics(sys.argv[1])
     rng = np.random.default_rng(2024)
     out = {}
     lens = [7, 64, 500, 3000, 20000]

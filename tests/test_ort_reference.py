@@ -22,9 +22,9 @@ pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not _OK, reason=f"genuine refe
 
 
 def _import_reference():
-    """the unmodified reference package: installed, or from baseline/_ref, or from /root/reference"""
+    """the unmodified reference package: installed, or from baseline/_ref"""
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    for extra in (None, os.path.join(root, "baseline", "_ref"), "/root/reference"):
+    for extra in (None, os.path.join(root, "baseline", "_ref")):
         if extra and os.path.isdir(extra) and extra not in sys.path:
             sys.path.insert(0, extra)
         try:
