@@ -49,6 +49,7 @@ extern "C" {
 #define OWW_WINDOW_ROWS         76   /* mel rows per embedding window          */
 #define OWW_EMBEDDING_DIM       96
 #define OWW_INIT_FEATURE_ROWS   41   /* rows AudioFeatures seeds the ring with */
+#define OWW_MAX_HEAD_FRAMES    120   /* rows AudioFeatures keeps (utils.py:170): the widest head window */
 #define OWW_MAX_HEAD_LAYERS      8
 
 /* embedding-CNN execution modes */
@@ -82,7 +83,9 @@ typedef struct oww_config {
 } oww_config;
 
 typedef struct oww_head_desc {
-    int32_t n_in;                              /* embedding frames read per prediction (model_inputs)  */
+    int32_t n_in;                              /* embedding frames read per prediction (model_inputs),
+                                                  1..OWW_MAX_HEAD_FRAMES: no wider window exists in the reference,
+                                                  and up to that every window fits the stream's feature ring      */
     int32_t n_layers;                          /* Linear layers (>=1, <= OWW_MAX_HEAD_LAYERS)          */
     int32_t dims[OWW_MAX_HEAD_LAYERS + 1];     /* dims[0] = n_in*96, dims[n_layers] = n_out            */
     int32_t layernorm;                         /* 1: LayerNorm(eps 1e-5) after every hidden Linear     */

@@ -403,6 +403,11 @@ int oww_add_head(oww_ctx* ctx, const oww_head_desc* desc, const float* h_blob, s
         return oww_fail(ctx, OWW_EUNSUPPORTED, "head has %d Linear layers (1..%d supported)", desc->n_layers, OWW_MAX_HEAD_LAYERS);
     if (desc->n_in < 1 || desc->dims[0] != desc->n_in * OWW_EMBEDDING_DIM)
         return oww_fail(ctx, OWW_EINVAL, "dims[0]=%d must equal n_in*96=%d", desc->dims[0], desc->n_in * OWW_EMBEDDING_DIM);
+    if (desc->n_in > OWW_MAX_HEAD_FRAMES)
+        // a chunk `back` rows before the newest reads ring rows count-back-n_in .. count-back-1 (mod feat_rows); with
+        // n_in + back > feat_rows the oldest alias newer ones.  feat_rows >= 120 + max_chunks keeps 120-row windows clear.
+        return oww_fail(ctx, OWW_EUNSUPPORTED, "head n_in=%d exceeds the reference's %d-row feature buffer",
+                        desc->n_in, OWW_MAX_HEAD_FRAMES);
     if (desc->final_act < 0 || desc->final_act > 4) return oww_fail(ctx, OWW_EINVAL, "bad final_act");
     if (ctx->heads.size() >= 16) return oww_fail(ctx, OWW_EUNSUPPORTED, "at most 16 heads per handle");
     Head h;

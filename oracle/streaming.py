@@ -28,6 +28,47 @@ def embeddings_of_clip(emb_weights, pcm, dtype=np.float32):
     return _emb.embed_windows(emb_weights, np.stack(wins), dtype)
 
 
+def stream_features(emb_weights, pcm, plan, feature_init, resets=None, dtype=np.float32):
+    """Every feature row one stream receives, computed in one CNN pass per segment instead of one per window.
+
+    pcm: the stream's samples (sum(plan) * 1280 of them); plan: chunks per call; feature_init: rows the stream starts
+    with; resets: {call index: init rows} - the stream is reset (``OracleAudioFeatures.reset``) just before that call.
+    The mel history of a segment is built as ``OracleAudioFeatures.__call__`` builds it: ones(76, 32), then per call the
+    mel of the last n*1280+480 samples (at most the segment's samples: 8n-3 rows on a fresh stream's first call, 8n after),
+    each call with its own -80 dB clamp.  The windows of the streaming state machine end at the history's end minus
+    multiples of 8, i.e. they start at rows 5, 13, 21, ...; the CNN's pooling strides total 8, so one
+    ``embedding.forward`` over history[5:] yields all of them.
+
+    Returns (rows, ends, starts): rows [N, 96] float32 in the order the stream's feature ring receives them, every
+    segment's init rows included; after call k the stream's buffer is rows[starts[k]:ends[k]] (before the reference's
+    120-row cap), so a head of n_in frames scores chunk i (0 = newest) of call k on rows[ends[k]-i-n_in : ends[k]-i]."""
+    resets = dict(resets or {})
+    pcm = np.asarray(pcm)
+    assert pcm.shape[0] == sum(plan) * CHUNK
+    bounds = sorted(set([0] + [k for k in resets if 0 < k < len(plan)])) + [len(plan)]
+    rows, ends, starts = [], [], []
+    n_rows, pos = 0, 0
+    for a, b in zip(bounds[:-1], bounds[1:]):
+        init = np.asarray(resets.get(a, feature_init), np.float32).reshape(-1, 96)
+        start = n_rows
+        rows.append(init)
+        n_rows += init.shape[0]
+        hist = [np.ones((WINDOW, 32), np.float32)]
+        seg0 = pos
+        for k in range(a, b):
+            pos += plan[k] * CHUNK
+            hist.append(_mel.melspectrogram(pcm[max(seg0, pos - plan[k] * CHUNK - TAIL):pos], dtype))
+        h = np.concatenate(hist)[5:]
+        emb = _emb.forward(emb_weights, h[None], dtype)[0]
+        assert emb.shape[0] == sum(plan[a:b])
+        rows.append(emb)
+        for k in range(a, b):
+            n_rows += plan[k]
+            ends.append(n_rows)
+            starts.append(start)
+    return np.concatenate(rows).astype(np.float32), np.array(ends), np.array(starts)
+
+
 class OracleAudioFeatures:
     def __init__(self, emb_weights, feature_init=None, init_noise=None, dtype=np.float32):
         self.w = emb_weights

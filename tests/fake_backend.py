@@ -6,6 +6,9 @@ import numpy as np
 
 from oracle import mel as omel, embedding as oemb, heads as oheads, streaming as ostream
 from openwakeword_b200 import weights as W
+from openwakeword_b200._native import NativeError
+
+MAX_HEAD_FRAMES = 120        # OWW_MAX_HEAD_FRAMES: the rows of the reference's feature buffer
 
 
 def unpack_embedding_blob(blob):
@@ -55,6 +58,9 @@ class FakeContext:
         self.emb = unpack_embedding_blob(np.asarray(blob, np.float32))
 
     def add_head(self, n_in, dims, layernorm, final_act, blob):
+        if n_in > MAX_HEAD_FRAMES:                       # oww_add_head's bound (include/owwb200.h)
+            raise NativeError(f"libowwb200 error -4: head n_in={n_in} exceeds the reference's "
+                              f"{MAX_HEAD_FRAMES}-row feature buffer")
         self.heads.append(unpack_head_blob(n_in, list(dims), layernorm, final_act, np.asarray(blob, np.float32)))
         return len(self.heads) - 1
 

@@ -140,6 +140,21 @@ def test_model_errors_match_reference(fake_ctx):
     assert m.get_parent_model_from_label("alexa_v0.1") == "alexa_v0.1"
 
 
+def test_model_rejects_heads_wider_than_the_feature_buffer(fake_ctx):
+    """oww_add_head bounds n_in by the reference's 120-row feature buffer (a wider window would read ring slots that
+    hold newer rows); the fake context keeps the same contract, so Model sees the same error on both."""
+    hdr = open(os.path.join(ROOT, "include", "owwb200.h")).read()
+    assert re.search(r"#define\s+OWW_MAX_HEAD_FRAMES\s+(\d+)", hdr).group(1) == str(fake_backend.MAX_HEAD_FRAMES) == "120"
+    wide = W.synthetic_head(n_in=121, hidden=8, seed=2)
+    with pytest.raises(_native.NativeError, match="n_in=121 exceeds the reference's 120-row feature buffer"):
+        owb.Model(wakeword_models=[{"name": "wide", "head": wide}], embedding_model_path=emb_weights())
+    fi = np.random.default_rng(0).normal(0, 1, (120, 96)).astype(np.float32)
+    m = owb.Model(wakeword_models=[{"name": "w120", "head": W.synthetic_head(n_in=120, hidden=8, seed=2)}],
+                  embedding_model_path=emb_weights(), feature_init=fi)
+    assert m.model_inputs["w120"] == 120
+    assert set(m.predict(np.zeros(1280, np.int16))) == {"w120"}
+
+
 def test_multi_stream_batch_equals_singles(fake_ctx):
     rng = np.random.default_rng(0)
     names = ["alexa_v0.1", "timer_v0.1"]

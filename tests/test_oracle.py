@@ -116,6 +116,41 @@ def test_heads_shapes_and_ranges():
     np.testing.assert_allclose(heads.forward(h, f16), torch.sigmoid(x).numpy(), atol=1e-6)
 
 
+def test_stream_features_matches_state_machine_call_by_call():
+    """streaming.stream_features (one CNN pass over a segment's mel history) against OracleAudioFeatures fed call by
+    call: 46 calls of 1, 2 and 3 chunks, a reset to 120 init rows after call 27, quiet / loud / silent / gated audio.
+    The embeddings each call appends and the 120-row feature_buffer must agree; the two differ only in NumPy's
+    summation order (measured worst 4.3e-6; gate ~5x)."""
+    rng = np.random.default_rng(4)
+    plan = [int(x) for x in rng.choice([1, 2, 3], 46)]
+    plan[:3] = [3, 1, 2]
+    plan[27:29] = [2, 1]                                     # a multi-chunk first call after the reset
+    n = sum(plan) * 1280
+    pcm = rng.normal(0, 3000, n) * np.repeat(rng.choice([0.0, 0.1, 1.0, 8.0], n // 4000 + 1), 4000)[:n]
+    pcm = np.clip(pcm, -32768, 32767).astype(np.int16)
+    fi = rng.normal(0, 1, (41, 96)).astype(np.float32)
+    fi2 = rng.normal(0, 1, (120, 96)).astype(np.float32)
+    rows, ends, starts = streaming.stream_features(emb_weights(), pcm, plan, fi, resets={27: fi2})
+    assert rows.shape == (41 + 120 + sum(plan), 96)
+    o = streaming.OracleAudioFeatures(emb_weights(), feature_init=fi)
+    pos, worst_emb, worst_buf = 0, 0.0, 0.0
+    for k, nch in enumerate(plan):
+        if k == 27:
+            o.reset(feature_init=fi2)
+        assert o(pcm[pos:pos + nch * 1280]) == nch * 1280
+        pos += nch * 1280
+        assert starts[k] == (0 if k < 27 else 41 + sum(plan[:27]))
+        assert ends[k] - starts[k] == (41 + sum(plan[:k + 1]) if k < 27 else 120 + sum(plan[27:k + 1]))
+        new = rows[ends[k] - nch:ends[k]]
+        worst_emb = max(worst_emb, float(np.abs(new - o.feature_buffer[-nch:]).max()))
+        buf = rows[max(starts[k], ends[k] - 120):ends[k]]
+        assert buf.shape == o.feature_buffer.shape
+        worst_buf = max(worst_buf, float(np.abs(buf - o.feature_buffer).max()))
+    print(f"stream_features vs OracleAudioFeatures: embeddings {worst_emb:.2e}, feature_buffer {worst_buf:.2e}")
+    assert worst_emb < 2e-5 and worst_buf < 2e-5
+    assert np.array_equal(rows[:41], fi) and np.array_equal(rows[starts[27]:starts[27] + 120], fi2)
+
+
 def test_first_chunk_yields_five_frames_and_ones_ring():
     """SURVEY.md F8 / Appendix D.1."""
     af = streaming.OracleAudioFeatures(emb_weights())
